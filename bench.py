@@ -71,7 +71,12 @@ def parse_args():
     ap.add_argument("--ref-budget-s", type=float, default=100.0, help="wall-clock target for all reference-arm steps together")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-file-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (per-read hit counts and rep_len, the hits of a fixed sample of reads) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs covers this repository's arm only (the reference arm's output is PAF/SAM text)")
+    return a
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -273,6 +278,40 @@ def gen_reads(L, idx, wl, n, read_len, seed, buf):
         L.mmb_synth_reads(idx, n, read_len, seed, wl["err"][0], wl["err"][1], wl["err"][2], buf.ctypes.data)
 
 
+DUMP_READS, DUMP_CIGAR_READS, DUMP_MAX_BYTES = 2048, 256, 64 << 20
+
+
+def collect_outputs(api, n_regs, regs, rep_len):
+    """What mm_map_batch() handed back, as float64 arrays: n_regs and rep_len of every read; for a fixed seeded sample of reads, every
+    field of their mm_reg1_t hits and of the mm_extra_t behind them, and the CIGAR words of the hits of the first DUMP_CIGAR_READS
+    sampled reads (hit h's words are cigar[hits.cigar_off[h]:][:hits.n_cigar[h]]; cigar_off is -1 for the other hits)"""
+    n = len(n_regs)
+    sample = np.sort(np.random.default_rng(0).permutation(n)[:DUMP_READS])
+    reg_fields = [f for f, _ in api.Reg1._fields_ if f != "p"]
+    ext_fields = [f for f, _ in api.Extra._fields_ if f != "capacity"]
+    cols = {f: [] for f in ["read"] + reg_fields + ext_fields + ["cigar_off"]}
+    cigar, n_words = [], 0
+    for k, i in enumerate(sample):
+        arr = C.cast(C.c_void_p(int(regs[i])), C.POINTER(api.Reg1)) if regs[i] else None
+        for j in range(int(n_regs[i])):
+            r = arr[j]
+            cols["read"].append(i)
+            for f in reg_fields:
+                cols[f].append(getattr(r, f))
+            ex = r.p.contents if r.p else None
+            for f in ext_fields:
+                cols[f].append(getattr(ex, f) if ex else 0)
+            cols["cigar_off"].append(n_words if ex and k < DUMP_CIGAR_READS else -1)
+            if ex and k < DUMP_CIGAR_READS:
+                cigar.append(np.ctypeslib.as_array((C.c_uint32 * ex.n_cigar).from_address(C.addressof(ex) + C.sizeof(api.Extra))).copy())
+                n_words += ex.n_cigar
+    out = {"n_regs": np.asarray(n_regs, dtype=np.float64), "rep_len": np.asarray(rep_len, dtype=np.float64), "sample_reads": sample.astype(np.float64),
+           "cigar": np.concatenate(cigar).astype(np.float64) if cigar else np.zeros(0)}
+    out.update({"hits." + ("as" if f == "as_" else f): np.asarray(v, dtype=np.float64) for f, v in cols.items()})
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES, "output dump above %d bytes" % DUMP_MAX_BYTES
+    return out
+
+
 def compare_outputs(a_path, b_path, log, sam=False):
     def lines(p):
         with open(p) as f:
@@ -437,15 +476,19 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def run_steps(n, resident):
+    dumped = {}
+
+    def run_steps(n, resident, dump=False):
         L.mmb_set_resident_reads(1 if resident else 0)
         bases, times = 0, []
-        for _ in range(n):
+        for it in range(n):
             t = time.perf_counter()
             n_regs, regs, rep = al.map_prepared(prepared)
             torch.cuda.synchronize()
             times.append(time.perf_counter() - t)
             bases = int(L.mmb_aligned_bases(n_reads, n_regs.ctypes.data, regs.ctypes.data, 1 if wl["kind"] == "ava" else 0))
+            if dump and it == n - 1:
+                dumped.update(collect_outputs(api, n_regs, regs, rep))
             al.free_batch(n_regs, regs)
         return bases, times
 
@@ -459,19 +502,21 @@ def main():
     L.mmb_launch_count_all(1)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    # --- timed region A: `value` (read bases resident in HBM; only the mm_map_batch calls are timed) ---
-    barrier()
-    bases, times_a = run_steps(a.steps, True)
-    barrier()
-    t_a = sum(times_a)
-    launches = int(L.mmb_launch_count_all(0))
-    # --- timed region B: `e2e` (host buffers in, results out) ---
-    barrier()
-    bases_b, times_b = run_steps(a.steps, False)
-    barrier()
-    t_b = sum(times_b)
-    d2h_bytes = int(L.mmb_last_d2h_bytes())
-    clocks = sampler.stop()
+    try:
+        # --- timed region A: `value` (read bases resident in HBM; only the mm_map_batch calls are timed) ---
+        barrier()
+        bases, times_a = run_steps(a.steps, True, dump=a.dump_outputs is not None)
+        barrier()
+        t_a = sum(times_a)
+        launches = int(L.mmb_launch_count_all(0))
+        # --- timed region B: `e2e` (host buffers in, results out) ---
+        barrier()
+        bases_b, times_b = run_steps(a.steps, False)
+        barrier()
+        t_b = sum(times_b)
+        d2h_bytes = int(L.mmb_last_d2h_bytes())
+    finally:  # the sampler is a child process: never leave it running
+        clocks = sampler.stop()
     # --- timed region C (rank 0's own figure is reported; every rank runs it so that the host is loaded as in production):
     #     `file_e2e` = mm_map_file(): FASTA in (page cache), PAF/SAM out (tmpfs) -- what the reference arm's number contains ---
     file_e2e = None
@@ -603,6 +648,10 @@ def main():
                 R.close()
         except Exception as e:  # the baseline is reported, never required for the GPU number
             line["cpu_baseline"] = {"value": None, "unit": "bases/s", "cores": n_threads_all, "kind": "reference", "sample": "failed: %r" % (e,)}
+    if a.dump_outputs:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for nm, arr in dumped.items():
+            np.save(os.path.join(a.dump_outputs, nm + ".npy"), arr)
     print(json.dumps(line))
     try:
         import shutil

@@ -2,6 +2,9 @@
 oracle/_ref/libminimap2_ref.so (the unmodified reference compiled by oracle/Makefile).
 Test infrastructure only -- never imported by minimap2_b200/."""
 import ctypes as C
+import gzip
+import hashlib
+import json
 import os
 import subprocess
 import numpy as np
@@ -55,6 +58,70 @@ def oracle():
 
 def have_ref():
     return os.path.exists(REF_SO)
+
+
+# ---------------- recorded reference results (tests/golden/ref/) ----------------
+# Tests that compare with the unmodified reference read what it computed from recordings keyed by their inputs, so that they run
+# (and never skip) where oracle/_ref cannot be built. MM2_RECORD_REF=1 runs the reference instead and rewrites the recording:
+#   MM2_RECORD_REF=1 python -m pytest tests -m "gpu or gpu_ext or not gpu"      (where oracle/_ref is built; GPU-side asserts may fail)
+RECORDED_DIR = os.path.join(ROOT, "tests", "golden", "ref")
+
+
+def file_digest(path):
+    with open(path, "rb") as f:
+        data = f.read()
+    if path.endswith(".gz"):
+        data = gzip.decompress(data)  # the gzip header carries a time stamp
+    return hashlib.sha256(data).hexdigest()
+
+
+def line_digest(line):
+    return hashlib.sha256(line.encode()).hexdigest()[:16]
+
+
+def recorded(key, produce):
+    """`produce()`'s JSON-able result, from the recording for `key` (a list of strings naming the inputs completely)"""
+    path = os.path.join(RECORDED_DIR, hashlib.sha256("\0".join(key).encode()).hexdigest()[:20] + ".json")
+    if os.environ.get("MM2_RECORD_REF") == "1":
+        os.makedirs(RECORDED_DIR, exist_ok=True)
+        with open(path, "w") as f:
+            json.dump({"key": key, "result": produce()}, f, separators=(",", ":"))
+            f.write("\n")
+    assert os.path.exists(path), "no recorded reference result for %r: record it with MM2_RECORD_REF=1 where oracle/_ref is built" % (key,)
+    with open(path) as f:
+        rec = json.load(f)
+    assert rec["key"] == key, (rec["key"], key)
+    return rec["result"]
+
+
+def cli_key(args, cwd=None):
+    """`args` with every input file replaced by its name and content digest (temporary paths differ from run to run)"""
+    key = []
+    for a in args:
+        p = os.path.join(cwd or "", a)
+        key.append("%s@%s" % (os.path.basename(a), file_digest(p)[:16]) if os.path.isfile(p) else a)
+    return key
+
+
+def ref_cli_lines(args, cwd=None):
+    """the reference CLI's stdout for `args` (no -t: the output does not depend on it) as line digests, SAM @PG dropped:
+    dict(args=, cwd=, lines=) for assert_same_lines"""
+    def produce():
+        p = subprocess.run([REF_BIN, "-t", "4"] + args, cwd=cwd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=1800)
+        assert p.returncode == 0, p.stderr.decode()[-2000:]
+        return [line_digest(l) for l in p.stdout.decode().splitlines() if not l.startswith("@PG")]
+    return dict(args=args, cwd=cwd, lines=recorded(["minimap2"] + cli_key(args, cwd), produce))
+
+
+def assert_same_lines(got, ref):
+    """`got` (output lines, SAM @PG dropped here) equals the reference output `ref` of ref_cli_lines, line by line"""
+    got = [l for l in got if not l.startswith("@PG")]
+    how = ("only digests of the reference's lines are stored; where oracle/_ref is built, `%s` (in %s) prints them"
+           % (" ".join([REF_BIN] + ref["args"]), ref["cwd"] or os.getcwd()))
+    assert len(got) == len(ref["lines"]), "%d output lines, the reference has %d (%s)" % (len(got), len(ref["lines"]), how)
+    for i, (l, d) in enumerate(zip(got, ref["lines"])):
+        assert line_digest(l) == d, "line %d differs from the reference's (%s):\ngot: %s" % (i, how, l[:600])
+    return len(got)
 
 
 def ref():

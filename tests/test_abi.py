@@ -44,18 +44,23 @@ def test_options_match_reference_presets():
     L.mm_set_opt.argtypes = [C.c_char_p, C.POINTER(api.IdxOpt), C.POINTER(api.MapOpt)]
     presets = [None, "map-ont", "lr", "ava-ont", "map-pb", "map10k", "ava-pb", "map-hifi", "map-ccs", "lr:hq", "lr:hqae", "map-iclr",
                "map-iclr-prerender", "asm5", "asm10", "asm20", "sr", "short", "splice", "splice:hq", "splice:sr", "cdna"]
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built")
-    R = O.ref()
-    R.mm_set_opt.argtypes = [C.c_char_p, C.POINTER(api.IdxOpt), C.POINTER(api.MapOpt)]
-    for p in presets:
-        io1, mo1, io2, mo2 = api.IdxOpt(), api.MapOpt(), api.IdxOpt(), api.MapOpt()
-        for lib_, io, mo in ((L, io1, mo1), (R, io2, mo2)):
-            lib_.mm_set_opt(None, C.byref(io), C.byref(mo))
-            if p is not None:
-                assert lib_.mm_set_opt(p.encode(), C.byref(io), C.byref(mo)) == 0
-        assert bytes(io1) == bytes(io2), p
-        assert bytes(mo1) == bytes(mo2), p
+
+    def set_opt(lib_, p):
+        io, mo = api.IdxOpt(), api.MapOpt()
+        lib_.mm_set_opt(None, C.byref(io), C.byref(mo))
+        if p is not None:
+            assert lib_.mm_set_opt(p.encode(), C.byref(io), C.byref(mo)) == 0
+        return [bytes(io).hex(), bytes(mo).hex()]
+
+    def produce():
+        R = O.ref()
+        R.mm_set_opt.argtypes = [C.c_char_p, C.POINTER(api.IdxOpt), C.POINTER(api.MapOpt)]
+        return [set_opt(R, p) for p in presets]
+    ref = O.recorded(["mm_set_opt"] + [str(p) for p in presets], produce)
+    for p, r in zip(presets, ref):
+        io, mo = set_opt(L, p)
+        assert io == r[0], p
+        assert mo == r[1], p
     io, mo = api.IdxOpt(), api.MapOpt()
     assert L.mm_set_opt(b"no-such-preset", C.byref(io), C.byref(mo)) == -1
     assert L.mm_set_opt(b"asm7", C.byref(io), C.byref(mo)) == -1

@@ -32,7 +32,6 @@ def cases():
     return m.CASES
 
 
-HAVE_REF = os.path.exists(O.REF_BIN)
 GOLDEN = ["inv_paf_cigar", "x3s_paf_cigar", "t2_paf_cigar"]  # MT-human/MT-orang goes through the .mmi test below
 
 
@@ -246,27 +245,26 @@ def emu_runs(emu_cli, tmp_path_factory):
         jobs[name] = (cases()[name], data, None)
     jobs["cig_overflow"] = (cases()["x3s_paf_cigar"], data, None, {"MM_B200_CIG_SHIFT": "6"})
     jobs["job_chunks"] = (cases()["x3s_paf_cigar"], data, None, {"MM_B200_JOB_CHUNK": "7"})
-    if HAVE_REF:
-        jobs["splice"] = (_splice_inputs(d), d, True)
-        jobs["splice_junc"] = (_splice_inputs(d, junc=True), d, True)
-        jobs["splice_spsc"] = (_splice_inputs(d, spsc=True), d, True)
-        jobs["high_occ"] = (_high_occ_inputs(d), d, True)
-        jobs["asm5"] = (_asm_inputs(d, "asm5", 0.004), d, True)
-        jobs["asm20"] = (_asm_inputs(d, "asm20", 0.03), d, True)
-        jobs["alt"] = (_alt_inputs(d), d, True)
-        jobs["ava"] = (_ava_inputs(d), d, True)
-        jobs["edge"] = (_edge_inputs(d), d, True)
-        jobs["rechain"] = (_rechain_inputs(d), d, True)
-        jobs["qstrand"] = (_qstrand_inputs(d), d, True)
-        jobs["sdust"] = (_sdust_inputs(d), d, True)
-        jobs["waves"] = (_many_waves_inputs(d), d, True)
-        jobs["multipart"] = (_multipart_inputs(d), d, True)
+    jobs["splice"] = (_splice_inputs(d), d, True)
+    jobs["splice_junc"] = (_splice_inputs(d, junc=True), d, True)
+    jobs["splice_spsc"] = (_splice_inputs(d, spsc=True), d, True)
+    jobs["high_occ"] = (_high_occ_inputs(d), d, True)
+    jobs["asm5"] = (_asm_inputs(d, "asm5", 0.004), d, True)
+    jobs["asm20"] = (_asm_inputs(d, "asm20", 0.03), d, True)
+    jobs["alt"] = (_alt_inputs(d), d, True)
+    jobs["ava"] = (_ava_inputs(d), d, True)
+    jobs["edge"] = (_edge_inputs(d), d, True)
+    jobs["rechain"] = (_rechain_inputs(d), d, True)
+    jobs["qstrand"] = (_qstrand_inputs(d), d, True)
+    jobs["sdust"] = (_sdust_inputs(d), d, True)
+    jobs["waves"] = (_many_waves_inputs(d), d, True)
+    jobs["multipart"] = (_multipart_inputs(d), d, True)
 
     def one(item):
         name, (args, cwd, with_ref), more_env = item[0], item[1][:3], (item[1][3] if len(item[1]) > 3 else {})
         ref = None
         if with_ref:
-            ref = subprocess.run([O.REF_BIN, "-t", "2"] + args, cwd=cwd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, check=True).stdout.decode().splitlines()
+            ref = O.ref_cli_lines(args, cwd)
         p = subprocess.run([emu_cli, "-t", "4"] + args, cwd=cwd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=1800, env=dict(env, **more_env))
         return name, dict(rc=p.returncode, err=p.stderr.decode()[-2000:], out=p.stdout.decode().splitlines(), ref=ref)
 
@@ -302,45 +300,40 @@ def test_emulated_many_job_chunks(emu_runs):
     assert r["out"] == exp
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_spliced_mapping_matches_reference(emu_runs):
     """-x splice end to end under the emulator (spliced kernel variant + splice branches of the driver) against the reference binary:
     two small cDNA reads, one per transcript strand"""
     r = emu_runs["splice"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) == 2
+    assert O.assert_same_lines(r["out"], r["ref"]) == 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_junction_annotation_matches_reference(emu_runs):
     """-x splice --junc-bed: mm_idx_bed_read on the index, the intron table on the device, junction flags derived per ksw_exts2 job
     in the kernel (mm_idx_bed_junc's window rule), for a genome without canonical splice signals"""
     r = emu_runs["splice_junc"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) == 2
+    assert O.assert_same_lines(r["out"], r["ref"]) == 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_splice_scores_match_reference(emu_runs):
     """-x splice --spsc: mm_idx_spsc_read2 on the index, per-strand score tables on the device, junc[] bytes assembled per ksw_exts2
     job in the kernel (mm_idx_spsc_get's window rule), KSW_EZ_SPLICE_SCORE on every spliced call"""
     r = emu_runs["splice_spsc"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) == 2
+    assert O.assert_same_lines(r["out"], r["ref"]) == 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_high_occurrence_seed_selection_matches_reference(emu_runs):
     """mm_seed_select (seed.c:56-96) on the device: a genome made mostly of copies of one 400 bp unit and -f 3 put most minimizers of
     every read above mid_occ, so the streak selection (heap of the lowest-occurrence seeds per stretch, max_max_occ cut, rep_len)
     decides which seeds are kept; -e 150 makes several seeds per stretch survive. Output equals the reference binary's."""
     r = emu_runs["high_occ"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 3
-    assert any("rl:i:" in l and "rl:i:0" not in l for l in r["ref"])  # the selection really masked something
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 3
+    assert any("rl:i:" in l and "rl:i:0" not in l for l in r["out"])  # the selection really masked something
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 @pytest.mark.parametrize("preset", ["asm5", "asm20"])
 def test_emulated_assembly_presets_match_reference(emu_runs, preset):
     """-x asm5 / asm20 (MM_F_RMQ: mg_lchain_rmq is the first chainer, map.c:275-276, followed by the bw_long re-chain of
@@ -348,99 +341,92 @@ def test_emulated_assembly_presets_match_reference(emu_runs, preset):
     reverse-complemented tail. Output equals the reference binary's."""
     r = emu_runs[preset]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 2
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_second_occurrence_cutoff_matches_reference(emu_runs):
     """-f INT,INT: the re-chaining pass of map.c:293-316 (seeds collected again with max_occ for reads left without a chain)"""
     r = emu_runs["rechain"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"]
-    assert any(l.startswith("in0\t") for l in r["ref"]) and any(l.startswith("in1\t") for l in r["ref"])  # mapped thanks to the second pass
+    O.assert_same_lines(r["out"], r["ref"])
+    assert any(l.startswith("in0\t") for l in r["out"]) and any(l.startswith("in1\t") for l in r["out"])  # mapped thanks to the second pass
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_query_strand_mode_matches_reference(emu_runs):
     """--qstrand end to end: anchors of reverse hits in other-strand coordinates (map.c:188-192), jobs that read the target
     complemented (MMB_JOB_T_COMP, universal kernel), flipped PAF coordinates and cs on that view (format.c:343-346,440-443)"""
     r = emu_runs["qstrand"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and sum(l.split("\t")[4] == "-" for l in r["ref"]) >= 2
+    O.assert_same_lines(r["out"], r["ref"])
+    assert sum(l.split("\t")[4] == "-" for l in r["out"]) >= 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_sdust_masking_matches_reference(emu_runs):
     """-T: symmetric DUST intervals from the host (hl_sdust), minimizers squeezed on the device before the occurrence filter"""
     r = emu_runs["sdust"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 2
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 2
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_many_alignment_waves_match_reference(emu_runs):
     """repeated z-drop splits: more replay / GPU waves than the scheduler used to allow (regression test for a fuzzing find)"""
     r = emu_runs["waves"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 1
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 1
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_alt_contigs_match_reference(emu_runs):
     """--alt (mm_idx_alt_read index.c:648-670, mm_mark_alt + the ALT-aware mm_hit_sort / mm_set_parent of hit.c:91-223 at
     map.c:321-324): reads from a region with an ALT haplotype; the ALT hits are down-weighted like the reference does."""
     r = emu_runs["alt"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 4
-    r0 = [l.split("\t") for l in r["ref"] if l.startswith("r0\t")]  # sampled from the ALT haplotype, yet the primary contig wins with MAPQ 60
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 4
+    r0 = [l.split("\t") for l in r["out"] if l.startswith("r0\t")]  # sampled from the ALT haplotype, yet the primary contig wins with MAPQ 60
     assert r0[0][5] == "chr0" and r0[0][11] == "60" and "tp:A:P" in r0[0] and r0[1][5] == "chr0_alt" and "tp:A:S" in r0[1]
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_all_vs_all_overlap_matches_reference(emu_runs):
     """-x ava-ont reads-vs-reads (skip_seed of map.c:78-100 with NO_DIAG / NO_DUAL on the device, occ_dist = 0 branch of the seed
     selection, ALL_CHAINS, no base-level alignment): five overlapping reads, alternating strands, names out of order"""
     r = emu_runs["ava"]
     assert r["rc"] == 0, r["err"]
-    assert r["out"] == r["ref"] and len(r["ref"]) >= 4
+    assert O.assert_same_lines(r["out"], r["ref"]) >= 4
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 @pytest.mark.parametrize("name,n_min", [("edge", 7), ("multipart", 3)])
 def test_emulated_cli_edge_cases_match_reference(emu_runs, name, n_min):
     """unmappable reads, gzipped FASTQ with comments in SAM (-a -y), several mini-batches; a multi-part index with --paf-no-hit"""
     r = emu_runs[name]
     assert r["rc"] == 0, r["err"]
-    strip = lambda ls: [l for l in ls if not l.startswith("@PG")]
-    assert strip(r["out"]) == strip(r["ref"]) and len(r["ref"]) >= n_min
+    assert O.assert_same_lines(r["out"], r["ref"]) >= n_min
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_mmi_files_are_interchangeable(emu_cli, tmp_path):
-    """mm_idx_dump / mm_idx_load (index.c:475-569): the reference maps with an index file written here and this library maps with one
-    written by the reference, both giving the recorded reference output (MT-human / MT-orang, the golden mt_paf_cigar case)"""
+    """mm_idx_dump / mm_idx_load (index.c:475-569): this library maps with an index file written by the reference (MT-human.ref.mmi,
+    `minimap2 -d` of the reference) and with its own, both giving the recorded reference output (MT-human / MT-orang, the golden
+    mt_paf_cigar case); where oracle/_ref is built, the reference also maps with the index written here"""
     data = os.path.join(GOLD, "data")
     exp = open(os.path.join(GOLD, "expected", "mt_paf_cigar.txt")).read().splitlines()
-    mine, theirs = str(tmp_path / "mine.mmi"), str(tmp_path / "ref.mmi")
+    mine, theirs = str(tmp_path / "mine.mmi"), os.path.join(data, "MT-human.ref.mmi")
     env = dict(os.environ, MM_B200_GROUPS="1")
     subprocess.run([emu_cli, "-t", "2", "-d", mine, os.path.join(data, "MT-human.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=env)
-    subprocess.run([O.REF_BIN, "-t", "2", "-d", theirs, os.path.join(data, "MT-human.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
     assert os.path.getsize(mine) == os.path.getsize(theirs)
-    out = subprocess.run([O.REF_BIN, "-t", "2", "-c", mine, os.path.join(data, "MT-orang.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE).stdout.decode().splitlines()
-    assert out == exp
-    out = subprocess.run([emu_cli, "-t", "2", "-c", theirs, os.path.join(data, "MT-orang.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=env, timeout=1200).stdout.decode().splitlines()
-    assert out == exp
+    if os.path.exists(O.REF_BIN):
+        out = subprocess.run([O.REF_BIN, "-t", "2", "-c", mine, os.path.join(data, "MT-orang.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE).stdout.decode().splitlines()
+        assert out == exp
+    for idx in (theirs, mine):
+        out = subprocess.run([emu_cli, "-t", "2", "-c", idx, os.path.join(data, "MT-orang.fa")], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=env, timeout=1200).stdout.decode().splitlines()
+        assert out == exp, idx
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 def test_emulated_spliced_extension_ignores_the_band(emu_cli):
     """ksw_exts2_sse takes no band (ksw2_exts2_sse.c:26-31). With -G 500 the driver's bandwidth (751) is smaller than the window of a right
     extension that runs on through a 766-bp intron; the spliced kernel used to clip the DP to that band and end the hit early (found by
     tests/cuda_emu/fuzz_cli.py --splice, seed 6009)."""
     data = os.path.join(GOLD, "data")
-    args = ["-t", "3", "-x", "splice", "-c", "--MD", "-C", "5", "-G", "500", os.path.join(data, "splice_G500_ref.fa"), os.path.join(data, "splice_G500_q.fa")]
-    got = subprocess.run([emu_cli] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=dict(os.environ, MM_B200_GROUPS="1"), timeout=1200)
-    ref = subprocess.run([O.REF_BIN] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=600)
+    args = ["-x", "splice", "-c", "--MD", "-C", "5", "-G", "500", os.path.join(data, "splice_G500_ref.fa"), os.path.join(data, "splice_G500_q.fa")]
+    got = subprocess.run([emu_cli, "-t", "3"] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, env=dict(os.environ, MM_B200_GROUPS="1"), timeout=1200)
     assert got.returncode == 0, got.stderr.decode()[-1000:]
-    assert got.stdout.decode().splitlines() == ref.stdout.decode().splitlines()
-    assert any("766N" in l for l in ref.stdout.decode().splitlines())
+    out = got.stdout.decode().splitlines()
+    O.assert_same_lines(out, O.ref_cli_lines(args))
+    assert any("766N" in l for l in out)

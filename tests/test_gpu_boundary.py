@@ -1,5 +1,5 @@
 """GPU: the drop-in boundary proven with the reference's OWN callers, unmodified, linked against libminimap2_b200.so
-(tests/boundary/build_boundary.py): example.c (mm_idx_reader_*, mm_mapopt_update, mm_tbuf_*, mm_map, kseq), main.c (the complete CLI incl.
+(tests/boundary/build_boundary.py, run by build() into oracle/_ref/boundary): example.c (mm_idx_reader_*, mm_mapopt_update, mm_tbuf_*, mm_map, kseq), main.c (the complete CLI incl.
 mm_write_sam_hdr, mm_map_file) and the Cython binding mappy (python/mappy.pyx + cmappy.h: Aligner, map with cs/MD, ThreadBuffer, fastx_read,
 seq, revcomp; several threads sharing one Aligner). Expected outputs were produced by the same callers linked against the reference library
 (tests/golden/make_boundary_golden.py)."""
@@ -11,10 +11,10 @@ import pytest
 import oracle_lib as O
 
 pytestmark = pytest.mark.gpu
-BUILD = os.path.join(O.ROOT, "tests", "boundary", "_build")
+BUILD = os.path.join(O.ORACLE_DIR, "_ref", "boundary")
 GOLD = os.path.join(O.ROOT, "tests", "golden")
 DATA = os.path.join(GOLD, "data")
-need = pytest.mark.skipif(not os.path.exists(os.path.join(BUILD, "example")), reason="tests/boundary/_build missing (built where /root/reference exists)")
+need = pytest.mark.skipif(not os.path.exists(os.path.join(BUILD, "example")), reason="oracle/_ref/boundary not built")
 
 
 @need

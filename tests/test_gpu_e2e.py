@@ -1,5 +1,6 @@
 """GPU end-to-end parity: the B200 mapper's CLI output vs the unmodified reference binary (oracle/_ref/minimap2) on the
-same inputs -- every PAF column and tag (NM ms AS nn tp cm s1 s2 de/dv zd rl cg) must match byte for byte."""
+same inputs -- every PAF column and tag (NM ms AS nn tp cm s1 s2 de/dv zd rl cg) must match byte for byte. The reference's
+output is read from its recording under tests/golden/ref (oracle_lib.recorded)."""
 import os
 import subprocess
 import numpy as np
@@ -19,40 +20,27 @@ def run(binary, args):
     return p.stdout.decode().splitlines()
 
 
-def compare(args, sam=False):
-    ref = run(O.REF_BIN, ["-t", "4"] + args)
-    got = run(MINE, ["-t", "8"] + args)
-    if sam:
-        ref = [l for l in ref if not l.startswith("@PG")]
-        got = [l for l in got if not l.startswith("@PG")]
-    assert len(ref) == len(got), (len(ref), len(got))
-    for i, (a, b) in enumerate(zip(ref, got)):
-        assert a == b, "line %d differs:\nref: %s\ngot: %s" % (i, a[:600], b[:600])
-    return len(ref)
+def compare(args):
+    return O.assert_same_lines(run(MINE, ["-t", "8"] + args), O.ref_cli_lines(args))
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_mt_paf():
     assert compare(["-c", os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")]) == 1
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_mt_sam_config0():
     """BASELINE.json configs[0]: minimap2 -a test/MT-human.fa test/MT-orang.fa"""
-    compare(["-a", os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")], sam=True)
+    compare(["-a", os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_mt_nocigar():
     compare([os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_inversion_pair():
     assert compare(["-c", os.path.join(DATA, "t-inv.fa"), os.path.join(DATA, "q-inv.fa")]) == 6
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("cfg", [dict(seed=1, glen=2_000_000, n=300, rlen=10000, err=0.10, rep=0.0, chim=0.0),
                                  dict(seed=2, glen=1_000_000, n=200, rlen=8000, err=0.12, rep=0.2, chim=0.1),
                                  dict(seed=3, glen=500_000, n=300, rlen=3000, err=0.05, rep=0.1, chim=0.05)])
@@ -66,7 +54,6 @@ def test_synthetic_map_ont(tmp_path, cfg):
     assert n >= cfg["n"] * 0.9
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("gap", [["-O4", "-E2"], ["-O6", "-E3"]])
 def test_single_affine_gap_cost(tmp_path, gap):
     """q == q2 and e == e2 select ksw_extz2 in the reference (align.c:360); here the dual-affine kernels run with equal terms"""
@@ -87,21 +74,18 @@ def _overlap_set(tmp_path, seed, glen=300_000, n=240, rlen=5000):
     return qf
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_ava_ont_overlaps(tmp_path):
     """BASELINE config 4 shape: all-vs-all overlap, skip_seed's name tests (NO_DIAG, NO_DUAL) evaluated on the device"""
     qf = _overlap_set(tmp_path, 31)
     assert compare(["-x", "ava-ont", qf, qf]) > 100
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_ava_with_cigar(tmp_path):
     """-X with base-level alignment: self-chain anchors carry MM_SEED_SELF into mm_align1 (align.c:760)"""
     qf = _overlap_set(tmp_path, 32, glen=150_000, n=100, rlen=4000)
     compare(["-x", "map-ont", "-X", "-c", qf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("strand", ["--for-only", "--rev-only"])
 def test_strand_restricted(tmp_path, strand):
     compare(["-c", strand, os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")])
@@ -113,10 +97,9 @@ def test_strand_restricted(tmp_path, strand):
     compare(["-x", "map-ont", "-c", strand, rf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
-@pytest.mark.parametrize("cfg", [dict(opts=["-x", "map-ont", "-c"], glen=20_000_000, n=1500, rlen=8000, err=0.10, rep=0.1, chim=0.05, sam=False),
-                                 dict(opts=["-x", "map-hifi", "-a"], glen=20_000_000, n=1000, rlen=12000, err=0.005, rep=0.1, chim=0.02, sam=True),
-                                 dict(opts=["-x", "ava-ont"], glen=1_500_000, n=800, rlen=6000, err=0.08, rep=0.0, chim=0.0, sam=False)])
+@pytest.mark.parametrize("cfg", [dict(opts=["-x", "map-ont", "-c"], glen=20_000_000, n=1500, rlen=8000, err=0.10, rep=0.1, chim=0.05),
+                                 dict(opts=["-x", "map-hifi", "-a"], glen=20_000_000, n=1000, rlen=12000, err=0.005, rep=0.1, chim=0.02),
+                                 dict(opts=["-x", "ava-ont"], glen=1_500_000, n=800, rlen=6000, err=0.08, rep=0.0, chim=0.0)])
 def test_scheduler_scale(tmp_path, cfg):
     """Batches large enough (>= 768 reads and >= 4 Mbases) for the scheduler to cut them into its 12 concurrent read groups -- the
     configuration the benchmark runs in: per-group streams and arenas, the device-slot gate, the shared host pool, K4 per group.
@@ -126,11 +109,5 @@ def test_scheduler_scale(tmp_path, cfg):
     rf, qf = str(tmp_path / "ref.fa"), str(tmp_path / "reads.fa")
     synth.write_fasta(rf, ["chr%d" % i for i in range(len(contigs))], contigs)
     synth.write_fasta(qf, ["read%d" % i for i in range(len(reads))], reads)
-    ava = cfg["opts"][-1] == "ava-ont"
-    ref = run(O.REF_BIN, ["-t", "32"] + cfg["opts"] + ([qf, qf] if ava else [rf, qf]))
-    got = run(MINE, ["-t", "16"] + cfg["opts"] + ([qf, qf] if ava else [rf, qf]))
-    if cfg["sam"]:
-        ref = [l for l in ref if not l.startswith("@PG")]; got = [l for l in got if not l.startswith("@PG")]
-    assert len(ref) == len(got) and len(ref) >= cfg["n"] * 0.5, (len(ref), len(got))
-    for i, (a, b) in enumerate(zip(ref, got)):
-        assert a == b, "line %d differs:\nref: %s\ngot: %s" % (i, a[:600], b[:600])
+    args = cfg["opts"] + ([qf, qf] if cfg["opts"][-1] == "ava-ont" else [rf, qf])
+    assert O.assert_same_lines(run(MINE, ["-t", "16"] + args), O.ref_cli_lines(args)) >= cfg["n"] * 0.5

@@ -5,20 +5,17 @@ binary, byte for byte."""
 import os
 import numpy as np
 import pytest
-import oracle_lib as O
 import synth
 from test_gpu_e2e import compare, DATA
 
 pytestmark = pytest.mark.gpu_ext
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("preset", ["asm5", "asm10", "asm20"])
 def test_mt_assembly_presets(preset):
     compare(["-x", preset, "-c", "--cs", os.path.join(DATA, "MT-human.fa"), os.path.join(DATA, "MT-orang.fa")])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("preset,div", [("asm5", 0.003), ("asm10", 0.02), ("asm20", 0.05)])
 def test_synthetic_contigs(tmp_path, preset, div):
     rng = np.random.default_rng(77)
@@ -44,7 +41,6 @@ def test_synthetic_contigs(tmp_path, preset, div):
     assert n >= len(asm)
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_alt_contigs(tmp_path):
     """--alt / --alt-drop (index.c:648-670, hit.c:91-223, map.c:321-324): ALT haplotypes of several regions next to the primary contigs"""
     rng = np.random.default_rng(5)
@@ -62,10 +58,9 @@ def test_alt_contigs(tmp_path):
     open(af, "w").write("".join(n + "\n" for n in names[2:]))
     n = compare(["-x", "map-ont", "-c", "--alt", af, rf, qf])
     assert n >= 400
-    compare(["-x", "map-ont", "-a", "--alt", af, "--alt-drop", "0.3", rf, qf], sam=True)
+    compare(["-x", "map-ont", "-a", "--alt", af, "--alt-drop", "0.3", rf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_junction_annotation_vs_reference(tmp_path):
     """-x splice --junc-bed (mm_idx_bed_read index.c:672-800; junction flags per ksw_exts2 call, align.c:638-643, derived in the
     kernel from the device intron table with mm_idx_bed_junc's window rule): transcripts over a genome where only a third of the
@@ -77,7 +72,7 @@ def test_junction_annotation_vs_reference(tmp_path):
     synth.write_fasta(rf, ["chr0"], [g]); synth.write_fasta(qf, ["tr%d" % i for i in range(len(reads))], reads)
     _write_bed(bed, introns, rng)
     assert compare(["-x", "splice", "-c", "--cs", "--junc-bed", bed, rf, qf]) >= 120
-    compare(["-x", "splice", "--junc-bed", bed, "--junc-bonus", "5", "-a", rf, qf], sam=True)
+    compare(["-x", "splice", "--junc-bed", bed, "--junc-bonus", "5", "-a", rf, qf])
 
 
 def test_splice_kernel_with_junction_table_matches_oracle():
@@ -94,7 +89,6 @@ def test_splice_kernel_with_junction_table_matches_oracle():
     ctx.close()
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 @pytest.mark.parametrize("extra", [["-f", "4,400", "-e", "0"], ["-f", "8,2000"]])
 def test_second_occurrence_cutoff(tmp_path, extra):
     """-f INT,INT (map.c:293-316): reads left without a chain by the first cutoff collect their seeds again with the second one"""
@@ -106,7 +100,6 @@ def test_second_occurrence_cutoff(tmp_path, extra):
     compare(["-c"] + extra + [rf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_splice_scores_vs_reference(tmp_path):
     """-x splice --spsc (mm_idx_spsc_read2 / mm_idx_spsc_get, index.c:963-1075; KSW_EZ_SPLICE_SCORE, align.c:688)"""
     from test_aligndriver_vs_ref import _spliced_set, _write_spsc
@@ -116,7 +109,7 @@ def test_splice_scores_vs_reference(tmp_path):
     synth.write_fasta(rf, ["chr0"], [g]); synth.write_fasta(qf, ["tr%d" % i for i in range(len(reads))], reads)
     _write_spsc(fn, g, introns, rng)
     assert compare(["-x", "splice", "-c", "--cs", "--spsc", fn, rf, qf]) >= 120
-    compare(["-x", "splice", "--spsc", fn, "--spsc-scale", "1", "--spsc0", "3", "-a", rf, qf], sam=True)
+    compare(["-x", "splice", "--spsc", fn, "--spsc-scale", "1", "--spsc0", "3", "-a", rf, qf])
 
 
 def test_splice_kernel_with_score_tables_matches_oracle():
@@ -133,7 +126,6 @@ def test_splice_kernel_with_score_tables_matches_oracle():
     ctx.close()
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_query_strand_mode(tmp_path):
     """--qstrand (main.c:252; map.c:188-192; align.c:780-783,815-818,875-878,899-901; format.c:343-346,440-443)"""
     contigs = synth.random_genome(500_000, 71, n_contigs=2, repeat_frac=0.1)
@@ -145,7 +137,6 @@ def test_query_strand_mode(tmp_path):
     compare(["--qstrand", rf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_sdust_masking(tmp_path):
     """-T 20 (mm_dust_minier, map.c:33-57): reads over a genome seeded with microsatellites and homopolymer runs"""
     rng = np.random.default_rng(17)
@@ -163,7 +154,6 @@ def test_sdust_masking(tmp_path):
     compare(["-x", "map-ont", "-T", "12", rf, qf])
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="oracle/_ref not built")
 def test_spliced_extension_ignores_the_band():
     """-x splice -G 500: the driver's bandwidth (751) is narrower than the window of a right extension that runs on through a 766-bp intron;
     ksw_exts2_sse takes no band (ksw2_exts2_sse.c:26-31). Device counterpart of tests/test_emu_e2e.py::test_emulated_spliced_extension_ignores_the_band

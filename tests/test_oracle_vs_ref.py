@@ -109,7 +109,8 @@ def test_radix_sort_tie_order():
 
 
 def make_anchors(rng, n_chain=3, n_noise=200, qlen=10000, span=15):
-    """anchors: x = rev<<63|rid<<32|rpos, y = span<<32|qpos; sorted by x with the reference's own sort"""
+    """anchors: x = rev<<63|rid<<32|rpos, y = span<<32|qpos; sorted by x with the oracle's radix sort (the reference's tie order:
+    test_sort128 and the recorded vectors of tests/test_golden.py pin it), so that callers need no reference build"""
     rows = []
     for c in range(n_chain):
         rid = int(rng.integers(0, 3)); rev = int(rng.integers(0, 2))
@@ -124,7 +125,7 @@ def make_anchors(rng, n_chain=3, n_noise=200, qlen=10000, span=15):
         rows.append(((int(rng.integers(0, 2)) << 63) | (int(rng.integers(0, 3)) << 32) | int(rng.integers(0, 200000)),
                      (span << 32) | int(rng.integers(span, qlen))))
     a = np.array(rows, dtype=np.uint64).reshape(-1, 2)
-    return O.ref_sort128(a)
+    return O.oracle_sort128(a)
 
 
 @pytest.mark.parametrize("seed", range(8))
